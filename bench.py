@@ -13,7 +13,7 @@ workloads and prints ONE JSON line:
                 (`--full-batch`; `--no-full-cycle` skips it, `--generator` makes it the headline instead).
 For each workload:
   value     faces/s with the input batches resident in HBM: CUDA-graph replay over `--slots` pipeline lanes, CUDA events
-            around exactly K steps, repeated over `--windows` back-to-back windows; the reported figure is the MEDIAN
+            around exactly K timed steps, split into `--windows` back-to-back windows; the reported figure is the MEDIAN
             window (min / max / relative spread alongside), max over ranks per window.  Inputs rotate over a set of
             batches larger than L2.  For N > 1 the NCCL all-gather of the final outputs runs INSIDE the timed region
             (on a communication stream, overlapping the next batch); `no_gather` repeats the measurement without it.
@@ -26,6 +26,9 @@ For each workload:
   parity    max errors of the timed configuration against the CPU oracle, checked in-run on one batch.
   cpu_baseline: `bench.py --impl reference` run as a child process on the host cores (so both arms share one code path
             and one thread-count choice).
+--dump-outputs DIR writes, after the timed steps, the outputs of the last timed step of each workload as float32 .npy
+files (headline: <key>.npy, full cycle: full_cycle_<key>.npy); inputs and weights are seeded, so two builds run with the
+same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -39,12 +42,14 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                              # the tree may be read-only: bench.py writes nothing there
 
 METRIC = "faces/sec encode->FLAME->render @224^2"
 UNIT = "faces/s"
 FLOPS_PER_FACE = {False: 0.941e9, True: 28.77e9}            # SURVEY.md §8d: encoder+FLAME ; + generator
 COMPULSORY_BYTES_PER_FACE = {False: 1.328e6, True: 2.532e6}
 CONSTANT_BYTES = {False: 38.0e6, True: 163.5e6}             # weights / FLAME constants read once per step
+DUMP_BYTES = 60_000_000                                     # --dump-outputs: all files together stay below 64 MB
 
 
 def load_peaks():
@@ -246,10 +251,13 @@ class Ctx:
 
 
 def timed_windows(cx, step, join, K, W, R):
-    """W warm-up steps, then R back-to-back windows of exactly K steps, each bracketed by CUDA events on the current
-    stream (which joins every lane / copy / communication stream before the closing event); barrier + synchronize on
-    both sides.  Returns the per-window ms, max over ranks."""
+    """W warm-up steps (indices 0..W-1), then exactly K timed steps (indices W..W+K-1) split into min(R, K) back-to-back
+    windows whose lengths differ by at most one, each bracketed by CUDA events on the current stream (which joins every
+    lane / copy / communication stream before the closing event); barrier + synchronize on both sides.  Returns the
+    per-window ms per step, max over ranks, and the window lengths."""
     import torch
+    R = max(1, min(R, K))
+    sizes = [K // R + (1 if r < K % R else 0) for r in range(R)]
     for i in range(W):
         step(i)
     join()
@@ -259,25 +267,37 @@ def timed_windows(cx, step, join, K, W, R):
     cx.barrier()
     for r in range(R):
         ev[r][0].record()
-        for _ in range(K):
+        for _ in range(sizes[r]):
             step(it)
             it += 1
         join()
         ev[r][1].record()
     cx.barrier()
-    t = torch.tensor([a.elapsed_time(b) for a, b in ev], device=cx.dev, dtype=torch.float64)
+    t = torch.tensor([a.elapsed_time(b) / n for (a, b), n in zip(ev, sizes)], device=cx.dev, dtype=torch.float64)
     if cx.dist is not None:
         cx.dist.all_reduce(t, op=cx.dist.ReduceOp.MAX)
-    return [float(x) for x in t.tolist()]
+    return [float(x) for x in t.tolist()], sizes
 
 
-def window_stats(ms, K):
+def window_stats(ms, sizes):
+    """ms: per-window ms per step."""
     med = statistics.median(ms)
-    return {"n": len(ms), "steps_per_window": K, "median_ms": med, "min_ms": min(ms), "max_ms": max(ms),
-            "rel_spread": (max(ms) - min(ms)) / med if med > 0 else None}
+    return {"n": len(ms), "steps_per_window": sizes, "median_ms_per_step": med, "min_ms_per_step": min(ms),
+            "max_ms_per_step": max(ms), "rel_spread": (max(ms) - min(ms)) / med if med > 0 else None}
 
 
-def run_workload(cx, args, B, generator, slots, R, with_cpu):
+def sample_outputs(outs, max_bytes, seed=0):
+    """Host float32 copies of one step's outputs (every array is batch-major).  When the whole batch exceeds
+    ``max_bytes``, every array keeps the same fixed, seeded subset of the faces, in batch order."""
+    import torch
+    B = next(iter(outs.values())).shape[0]
+    per_face = sum(t[0].numel() * 4 for t in outs.values())
+    n = min(B, max(1, max_bytes // per_face))
+    idx = torch.randperm(B, generator=torch.Generator().manual_seed(seed))[:n].sort().values
+    return {k: t[idx.to(t.device)].float().cpu().numpy() for k, t in outs.items()}
+
+
+def run_workload(cx, args, B, generator, slots, R, with_cpu, dump_bytes=0):
     """Measure one workload (device-resident, e2e, ± gather for N > 1, kernel breakdown, parity).  Returns a dict."""
     import torch
     import smirk_b200
@@ -321,20 +341,22 @@ def run_workload(cx, args, B, generator, slots, R, with_cpu):
         cx.last = pipe.run_host(host_imgs[i % Rset], i, host_masks[i % Rset] if generator else None, keys)
 
     out = {"batch": B, "launches_per_step": int(rec["launches"])}
-    faces = B * world * K
+    faces = B * world
     gather_keys = pipe.enable_gather(keys, backend=args.gather_backend) if (world > 1 and not args.no_gather) else ()
     sampler = ClockSampler(cx.local)
     if rank == 0:
         sampler.start()
-    ms = timed_windows(cx, dev_step, pipe.join, K, W, R)
+    ms, sizes = timed_windows(cx, dev_step, pipe.join, K, W, R)
     out["clocks"] = sampler.stop() if rank == 0 else None
-    out["windows"] = window_stats(ms, K)
-    out["ms_per_step"] = out["windows"]["median_ms"] / K
-    out["value"] = faces / (out["windows"]["median_ms"] / 1e3)
+    if dump_bytes and rank == 0:                # the lane of the last timed step still holds its outputs
+        out["dump"] = sample_outputs(pipe.capture(B, (W + K - 1) % pipe.slots)["out"], dump_bytes)
+    out["windows"] = window_stats(ms, sizes)
+    out["ms_per_step"] = out["windows"]["median_ms_per_step"]
+    out["value"] = faces / (out["ms_per_step"] / 1e3)
     h2d, d2h = pipe.bytes_per_step(B, keys)
-    ms2 = timed_windows(cx, host_step, pipe.join, K, W, max(3, R // 2))
+    ms2, sizes2 = timed_windows(cx, host_step, pipe.join, K, W, R)
     out["e2e"] = {"value": faces / (statistics.median(ms2) / 1e3), "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                  "ms_per_step": statistics.median(ms2) / K, "windows": window_stats(ms2, K),
+                  "ms_per_step": statistics.median(ms2), "windows": window_stats(ms2, sizes2),
                   "api": "SmirkPipeline.run_host (pinned host in/out, %d lanes, copies on their own streams)" % pipe.slots,
                   "host_checksum": float(cx.last["params"].double().abs().sum())}          # touches the host result
     if gather_keys:
@@ -347,9 +369,9 @@ def run_workload(cx, args, B, generator, slots, R, with_cpu):
         if pipe._gather_backend == "p2p" and isinstance(p2p, dict):
             out["gather"]["form"] = "packed: one staging copy, one push per peer, lane released after the pack" if p2p.get("pack") else "direct: one push per (output, peer)"
         pipe.enable_gather(())
-        ms3 = timed_windows(cx, dev_step, pipe.join, K, W, max(3, R // 2))
-        ms4 = timed_windows(cx, host_step, pipe.join, K, W, max(3, R // 2))
-        out["no_gather"] = {"value": faces / (statistics.median(ms3) / 1e3), "ms_per_step": statistics.median(ms3) / K,
+        ms3, _ = timed_windows(cx, dev_step, pipe.join, K, W, R)
+        ms4, _ = timed_windows(cx, host_step, pipe.join, K, W, R)
+        out["no_gather"] = {"value": faces / (statistics.median(ms3) / 1e3), "ms_per_step": statistics.median(ms3),
                             "e2e_value": faces / (statistics.median(ms4) / 1e3)}
 
     if rank != 0:
@@ -451,7 +473,7 @@ def main():
     ap.add_argument("--full-batch", type=int, default=256, help="faces per GPU per step of the full-cycle workload (configs[2]/[4] = 256)")
     ap.add_argument("--generator", action="store_true", help="make the full cycle (with SmirkGenerator) the headline workload at --batch")
     ap.add_argument("--no-full-cycle", action="store_true", help="skip the extra full_cycle block")
-    ap.add_argument("--windows", type=int, default=21, help="back-to-back repeats of the K-step timed window (median reported)")
+    ap.add_argument("--windows", type=int, default=1, help="split the K timed steps into this many back-to-back windows (median reported)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-gather", action="store_true", help="N > 1: leave the NCCL all-gather of the outputs out of the timed region")
@@ -465,9 +487,18 @@ def main():
                     help="encoder arithmetic.  tf32x3: tcgen05 tensor cores with error-compensated 3xTF32 products (fp32-equivalent; "
                          "the parity path and the default); tf32: plain TF32 tensor cores (the reference's cuDNN default); "
                          "fp32: exact fp32 CUDA cores.  The generator runs TF32 tcgen05 unless fp32 is chosen.")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the outputs of the last timed step of each workload to DIR/<name>.npy (float32, "
+                         "under 64 MB in all: a fixed, seeded subset of the faces when a batch is larger; bench_outputs/ is git-ignored)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "smirk_b200":
+        ap.error("--dump-outputs applies to the product arm")
     if args.profile_out:
         args.profile_out = os.path.abspath(args.profile_out)
+    if args.dump_outputs:
+        args.dump_outputs = os.path.abspath(args.dump_outputs)
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -502,10 +533,13 @@ def main():
         torch.cuda.synchronize(cx.dev)
     cx.barrier = barrier
 
-    head = run_workload(cx, args, args.batch, args.generator, args.slots, max(1, args.windows), with_cpu=(world == 1 and not args.no_cpu_baseline))
+    with_full = not args.generator and not args.no_full_cycle
+    dump_bytes = DUMP_BYTES // (2 if with_full else 1) if args.dump_outputs else 0
+    head = run_workload(cx, args, args.batch, args.generator, args.slots, max(1, args.windows), with_cpu=(world == 1 and not args.no_cpu_baseline),
+                        dump_bytes=dump_bytes)
     full = None
-    if not args.generator and not args.no_full_cycle:
-        full = run_workload(cx, args, args.full_batch, True, args.full_slots, max(1, min(args.windows, 5)), with_cpu=False)
+    if with_full:
+        full = run_workload(cx, args, args.full_batch, True, args.full_slots, max(1, args.windows), with_cpu=False, dump_bytes=dump_bytes)
 
     if rank == 0:
         B, K = args.batch, args.steps
@@ -522,7 +556,7 @@ def main():
                        "global_batch": B * world,
                        "faces_per_gpu_per_step": B, "image": "224x224 RGB fp32", "parallelism": "frame-shard dp%d" % world,
                        "l2_policy": "inputs rotate over a set of batches > 126 MB L2 (160 MB)",
-                       "timing": "median of %d back-to-back windows of exactly %d steps (CUDA events, max over ranks per window)" % (head["windows"]["n"], K),
+                       "timing": "%d timed steps in %d back-to-back windows, median window (CUDA events, max over ranks per window)" % (K, head["windows"]["n"]),
                        "execution": "CUDA graph replay, %d kernels per step, %d-lane software pipeline over consecutive steps" % (head["launches_per_step"], args.slots),
                        "host_affinity": affinity},
             "windows": head["windows"],
@@ -543,6 +577,12 @@ def main():
                 if k in full:
                     fc[k] = full[k]
             line["full_cycle"] = fc
+        if args.dump_outputs:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for prefix, res in (("", head), ("full_cycle_", full)):
+                for k, a in (res or {}).get("dump", {}).items():
+                    np.save(os.path.join(args.dump_outputs, prefix + k + ".npy"), a)
         print(json.dumps(line), flush=True)
     if cx.dist is not None:
         cx.dist.destroy_process_group()

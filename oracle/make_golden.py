@@ -23,6 +23,17 @@ GOLD = os.path.join(HERE, "..", "tests", "golden")
 N = lambda t: t.detach().cpu().numpy()
 
 
+def savez_lzma(path, **arrays):
+    """Like np.savez_compressed, with LZMA members (np.load reads them): keeps render.npz under 1 MB."""
+    import io
+    import zipfile
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as z:
+        for k, a in arrays.items():
+            buf = io.BytesIO()
+            np.save(buf, a)
+            z.writestr(k + ".npy", buf.getvalue())
+
+
 def main():
     root = synth_assets.materialize(os.path.join(tempfile.gettempdir(), "smk_assets_golden"))
     with ref_harness.reference(root) as R, torch.no_grad():
@@ -59,12 +70,12 @@ def main():
         from oracle import render_ref
         rr = render_ref.render_forward_ref(render_ref.RenderConstants(root), fr["vertices"], pr["cam"])
         assert torch.equal(ro["transformed_vertices"], rr["transformed_vertices"])
-        np.savez_compressed(os.path.join(GOLD, "render.npz"),
-                            vertices=N(fr["vertices"]), cam=N(pr["cam"]),
-                            rendered_img=N(ro["rendered_img"]), transformed_vertices=N(ro["transformed_vertices"]),
-                            landmarks_fan=N(ro["landmarks_fan"]), landmarks_mp=N(ro["landmarks_mp"]),
-                            pix_to_face=N(rr["pix_to_face"]).astype(np.int32), bary=N(rr["bary"]),
-                            faces=N(rend.faces[0]).astype(np.int16))
+        savez_lzma(os.path.join(GOLD, "render.npz"),
+                   vertices=N(fr["vertices"]), cam=N(pr["cam"]),
+                   rendered_img=N(ro["rendered_img"]), transformed_vertices=N(ro["transformed_vertices"]),
+                   landmarks_fan=N(ro["landmarks_fan"]), landmarks_mp=N(ro["landmarks_mp"]),
+                   pix_to_face=N(rr["pix_to_face"]).astype(np.int32), bary=N(rr["bary"]),
+                   faces=N(rend.faces[0]).astype(np.int16))
         # ---- Generator --------------------------------------------------------------------------
         gen = R.SmirkGenerator(in_channels=6, out_channels=3, init_features=32, res_blocks=5).eval()
         gen.load_state_dict(synth_inputs.random_state_dict(gen.state_dict(), seed=7))

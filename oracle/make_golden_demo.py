@@ -1,9 +1,17 @@
-"""ORACLE — TEST INFRASTRUCTURE ONLY.  Generates tests/golden/demo.npz by running the REFERENCE's own, unmodified
-``demo.py`` (/root/reference) with the reference's own classes on the CPU — third-party pieces (timm, pytorch3d, skimage,
-mediapipe) replaced by the stand-ins of oracle/ref_harness.py and tests/dropin_support.py — on the synthetic input image
-and synthetic checkpoint of tests/dropin_support.py.  Re-run in the build container: ``python -m oracle.make_golden_demo``.
+"""ORACLE — TEST INFRASTRUCTURE ONLY.  Generates tests/golden/demo.npz with the REFERENCE's own classes on the CPU —
+third-party pieces (timm, pytorch3d, skimage, mediapipe) replaced by the stand-ins of oracle/ref_harness.py and
+tests/dropin_support.py — on the synthetic input image and synthetic checkpoint of tests/dropin_support.py.  Needs a
+reference checkout (``SMIRK_REFERENCE``): ``python -m oracle.make_golden_demo``.
 
-Stored: the grid the script writes (demo.py:170-182) without ``--use_smirk_generator`` (cropped image | rendered mesh).
+Stored:
+  grid            the grid the reference's own, unmodified ``demo.py`` writes (demo.py:170-182) without
+                  ``--use_smirk_generator`` (cropped image | rendered mesh);
+  grid_generator  the grid tests/demo_flow.py writes with ``--use_smirk_generator`` (cropped image | rendered mesh |
+                  SmirkGenerator output) when its ``src.*`` imports resolve to the reference's classes; its masking step
+                  is the CPU oracle (tests/dropin_support.py), as in the test that compares against it;
+  generator_sampled_faces_indices, generator_barycentric_coords
+                  the masking samples that run drew.  The draws depend on the last bits of the face weights, which vary
+                  with the CPU, so the test replays these instead of drawing its own.
 """
 import os
 import subprocess
@@ -26,14 +34,22 @@ def main():
     work = tempfile.mkdtemp(prefix="smk_demo_golden_")
     root = synth_assets.materialize(os.path.join(work, "assets_root"))
     img = ds.synthetic_image(os.path.join(work, "face.png"))
-    ck = ds.write_checkpoint(os.path.join(work, "ck.pt"), with_generator=False)
-    out = os.path.join(work, "out")
-    subprocess.check_call([sys.executable, os.path.join(ROOT, "tests", "dropin_support.py"), "--mode", "reference", "--script",
-                           os.path.join(ref_harness.REF, "demo.py"), "--cwd", root, "--", "--input_path", img, "--device", "cpu",
-                           "--checkpoint", ck, "--out_path", out])
-    grid = cv2.imread(os.path.join(out, "face.png"))
-    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "demo.npz"), grid=grid)
-    print("demo.npz:", grid.shape, "rendered coverage %.3f" % float((grid[:, 224:] > 0).any(-1).mean()))
+    grids, dump = {}, os.path.join(work, "dump.pt")
+    for key, script, generator in (("grid", os.path.join(ref_harness.REF, "demo.py"), False),
+                                   ("grid_generator", os.path.join(ROOT, "tests", "demo_flow.py"), True)):
+        ck = ds.write_checkpoint(os.path.join(work, key + ".pt"), with_generator=generator)
+        out = os.path.join(work, "out_" + key)
+        subprocess.check_call([sys.executable, os.path.join(ROOT, "tests", "dropin_support.py"), "--mode", "reference", "--script", script,
+                               "--reference-root", ref_harness.REF, "--cwd", root, "--", "--input_path", img, "--device", "cpu",
+                               "--checkpoint", ck, "--out_path", out] + (["--use_smirk_generator", "--dump", dump] if generator else []))
+        grids[key] = cv2.imread(os.path.join(out, "face.png"))
+    import torch
+    t = torch.load(dump)
+    grids["generator_sampled_faces_indices"] = t["sampled_faces_indices"].numpy().astype(np.int32)
+    grids["generator_barycentric_coords"] = t["barycentric_coords"].numpy().astype(np.float32)
+    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "demo.npz"), **grids)
+    print("demo.npz:", {k: g.shape for k, g in grids.items()},
+          "rendered coverage %.3f" % float((grids["grid"][:, 224:] > 0).any(-1).mean()))
 
 
 if __name__ == "__main__":

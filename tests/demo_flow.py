@@ -1,8 +1,8 @@
-"""TEST INFRASTRUCTURE — the single-image flow of the reference's ``demo.py`` restated for machines that have a GPU but
-no reference checkout (the GPU box): same steps, same module names — it imports the hot-path classes from the names the
-reference uses (``src.smirk_encoder`` ...), which ``python -m smirk_b200.dropin`` aliases to smirk_b200 — and writes the
-same grid image.  Each block cites the demo.py lines it follows.  The unmodified script itself is exercised in the build
-container by tests/test_dropin_demo.py::test_unmodified_demo_script_runs_on_the_dropin_classes.
+"""TEST INFRASTRUCTURE — the single-image flow of the reference's ``demo.py`` restated so that it runs without a
+reference checkout: same steps, same module names — it imports the hot-path classes from the names the reference uses
+(``src.smirk_encoder`` ...), which ``python -m smirk_b200.dropin`` aliases to smirk_b200 — and writes the same grid
+image.  Each block cites the demo.py lines it follows.  tests/test_dropin_demo.py runs it on the GPU and, with the CPU
+oracle in place of the native calls, without one.
 
     python -m smirk_b200.dropin tests/demo_flow.py --input_path x.png --checkpoint ck.pt --out_path out [--use_smirk_generator]
 """
@@ -28,6 +28,8 @@ if __name__ == "__main__":
     ap.add_argument("--out_path", default="output")
     ap.add_argument("--use_smirk_generator", action="store_true")
     ap.add_argument("--dump", default=None, help="also save the tensors of the run here (.pt), for stage-wise checks")
+    ap.add_argument("--coords", default=None, help="masking samples (.npz: sampled_faces_indices, barycentric_coords) to use "
+                                                   "instead of drawing them, e.g. those of another run's --dump")
     args = ap.parse_args()
 
     # demo.py:54-59 — encoder + checkpoint ingest (keys carry a `smirk_encoder.` prefix)
@@ -80,6 +82,9 @@ if __name__ == "__main__":
         o = u + v > 1
         u[o], v[o] = 1 - u[o], 1 - v[o]
         bary = torch.stack((1 - (u + v), u, v), 1)[None]
+        if args.coords:                                             # the draws depend on the last bits of the weights
+            c = np.load(args.coords)
+            idx, bary = torch.from_numpy(c["sampled_faces_indices"]).long(), torch.from_numpy(c["barycentric_coords"]).float()
         npoints, _ = masking.mesh_based_mask_uniform_faces(tv, flame.faces_tensor, face_probabilities, mask_ratio=0.05,
                                                            coords={"sampled_faces_indices": idx, "barycentric_coords": bary})
         rbound = torch.tensor([num // 2])
@@ -89,7 +94,8 @@ if __name__ == "__main__":
         smirk_generator_input = torch.cat([rendered_img, masked_img], dim=1)
         reconstructed_img = smirk_generator(smirk_generator_input)
         grid = torch.cat([grid, reconstructed_img], dim=3)
-        dump.update(generator_input=smirk_generator_input, reconstructed_img=reconstructed_img, npoints=npoints)
+        dump.update(generator_input=smirk_generator_input, reconstructed_img=reconstructed_img, npoints=npoints,
+                    sampled_faces_indices=idx, barycentric_coords=bary)
 
     grid_numpy = (grid.squeeze(0).permute(1, 2, 0).detach().cpu().numpy() * 255.0).astype(np.uint8)   # demo.py:170-182
     grid_numpy = cv2.cvtColor(grid_numpy, cv2.COLOR_BGR2RGB)

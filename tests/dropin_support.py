@@ -8,9 +8,12 @@ synthetic input image, and a subprocess runner with three modes:
   dropin         ``python -m smirk_b200.dropin <script>``: the four hot-path modules replaced by smirk_b200 (needs a GPU)
   dropin-oracle  like dropin, but the native forwards of the smirk_b200 classes are patched HERE, in test code, to
                  evaluate the CPU oracle: exercises the drop-in surface (aliasing, constructors, checkpoint ingest,
-                 dict keys, attribute access from the unmodified script) on a machine without a GPU.  Never shipped.
+                 dict keys, attribute access from the script) on a machine without a GPU.  Never shipped.
 
-    python tests/dropin_support.py --mode reference --script /root/reference/demo.py --cwd <asset root> -- <script args>
+In the reference and dropin-oracle modes the smirk_b200.masking calls of tests/demo_flow.py evaluate the CPU oracle too.
+
+    python tests/dropin_support.py --mode reference --script <reference checkout>/demo.py --cwd <asset root> -- <script args>
+    python tests/dropin_support.py --mode dropin-oracle --script tests/demo_flow.py --cwd <asset root> -- <script args>
 """
 import argparse
 import os
@@ -154,19 +157,40 @@ def patch_native_with_oracle(asset_root):
     L.require_cuda = lambda t, name: None
 
 
+def patch_masking_with_oracle():
+    """The three smirk_b200.masking calls tests/demo_flow.py makes, evaluated by the CPU oracle (test code only), so the
+    flow's generator branch runs on a machine without a GPU — on the drop-in classes and on the reference's alike."""
+    import smirk_b200.masking as M
+    from oracle import masking_ref
+
+    def face_weights(tv, faces, face_probabilities):
+        return masking_ref.face_probabilities_ref(tv.float(), faces, face_probabilities.float())
+
+    def mesh_based_mask_uniform_faces(tv, faces, face_probabilities, mask_ratio=0.1, coords=None, IMAGE_SIZE=224):
+        idx, bary = coords["sampled_faces_indices"], coords["barycentric_coords"]
+        return masking_ref.points_from_coords_ref(tv.float(), faces, idx, bary, IMAGE_SIZE), coords
+
+    def masking_from_points(img, mask, npoints, rbound, wr=15, rendered_mask=None, flame_faces=None, **kw):
+        extra = img * masking_ref.point_mask_ref(npoints, rbound, img.shape[-1])
+        return masking_ref.masking_ref(img, mask, extra, wr, rendered_mask=rendered_mask)
+
+    M.face_weights, M.mesh_based_mask_uniform_faces, M.masking_from_points = face_weights, mesh_based_mask_uniform_faces, masking_from_points
+
+
 # ------------------------------------------------------------------------------------------------ runner
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--mode", required=True, choices=["reference", "dropin", "dropin-oracle"])
     ap.add_argument("--script", required=True)
     ap.add_argument("--cwd", required=True, help="asset root (the scripts use relative asset paths)")
+    ap.add_argument("--reference-root", default=None, help="checkout whose `src` package the script imports (default: the script's directory)")
     ap.add_argument("--seed", type=int, default=1234)
     ap.add_argument("rest", nargs=argparse.REMAINDER)
     a = ap.parse_args()
     rest = a.rest[1:] if a.rest and a.rest[0] == "--" else a.rest
     import torch
     sys.dont_write_bytecode = True
-    ref_root = os.path.dirname(os.path.abspath(a.script))
+    ref_root = os.path.abspath(a.reference_root or os.path.dirname(os.path.abspath(a.script)))
     install_third_party_stubs()
     os.chdir(a.cwd)
     if a.mode == "reference":
@@ -178,16 +202,19 @@ def main():
         dropin.install(ref_root)
         if a.mode == "dropin-oracle":
             patch_native_with_oracle(a.cwd)
-    # The scripts draw their masking samples from torch's global RNG (masking.py:160-162,84-96; demo.py:151-152) after
-    # building the models, whose constructors consume a class-dependent number of draws.  Re-seed at the first masking
-    # call so the reference classes and the drop-in classes see the same sample stream.
-    import src.utils.masking as M
-    load_prob = M.load_probabilities_per_FLAME_triangle
+    if a.mode != "dropin":
+        patch_masking_with_oracle()
+    # The reference's demo.py draws its masking samples from torch's global RNG (masking.py:160-162,84-96; demo.py:151-152)
+    # after building the models, whose constructors consume a class-dependent number of draws.  Re-seed at the first
+    # masking call so the reference classes and the drop-in classes see the same sample stream.
+    if os.path.isfile(os.path.join(ref_root, "src", "utils", "masking.py")):
+        import src.utils.masking as M
+        load_prob = M.load_probabilities_per_FLAME_triangle
 
-    def seeded_load(*args, **kw):
-        torch.manual_seed(a.seed)
-        return load_prob(*args, **kw)
-    M.load_probabilities_per_FLAME_triangle = seeded_load
+        def seeded_load(*args, **kw):
+            torch.manual_seed(a.seed)
+            return load_prob(*args, **kw)
+        M.load_probabilities_per_FLAME_triangle = seeded_load
     sys.argv = [a.script] + rest
     with torch.no_grad():
         runpy.run_path(a.script, run_name="__main__")
